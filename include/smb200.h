@@ -83,14 +83,6 @@ enum {
     SMB_OPT_POW_SPECIALISE = 0,
     /* Bytes per staging chunk of the host-operand pipeline (default 64 MiB). */
     SMB_OPT_STAGE_CHUNK_BYTES = 1,
-    /* Dense-stream kernels: cap the grid at this many CTAs per SM (0 = library default: one tile
-     * per CTA).  For the table-driven pow kernels the value counts consecutive TILES PER CTA
-     * instead (0 = default: 8 for f32, 32 for f64). */
-    SMB_OPT_CONTIG_VARIANT = 2,
-    /* Broadcast kernel: 1 = stage a small reused operand in shared memory (cp.async.bulk);
-     * 0 (default) = read it through L1/L2, which measured faster on B200; 2 = also disable
-     * the register-tiled outer kernel (A/B comparisons). */
-    SMB_OPT_BCAST_VARIANT = 3,
     /* Test hook: 1 = take the 64-bit index path (results beyond 2^31 elements) for every
      * broadcast launch, so it can be exercised on small shapes. */
     SMB_OPT_FORCE_WIDE_INDEX = 4,
@@ -110,30 +102,14 @@ enum {
      * (default 32 MiB). */
     SMB_OPT_SHARD_MIN_BYTES = 7,
     /* Device set: an operand several devices read (a broadcast row, an outer-product factor) is
-     * copied to each device per call when it is at most this large (default 64 MiB); a larger shared
-     * operand makes the operator run on one device. */
+     * kept as a read-mostly duplicate on each device when it is at most this large (default 64 MiB): the
+     * driver keeps a read-only copy per device and invalidates them on any write, raw host writes
+     * included.  A larger shared operand makes the operator run on one device. */
     SMB_OPT_REPLICATE_MAX_BYTES = 8,
     /* Pool high-water mark: when more than this many freed bytes sit cached, smb_free returns the
      * largest blocks to the driver (default 64 GiB; negative: never). */
-    SMB_OPT_POOL_MAX_CACHED_BYTES = 9,
-    /* Table-driven pow kernels: how many CTAs at the END of the grid own a single tile (they fill the
-     * ragged end the multi-tile CTAs leave).  0 (default): none -- measured no gain on B200. */
-    SMB_OPT_POW_TAIL_CTAS = 10,
-    /* Fused chains with a pow step and at most 3 leaves (sm::pow(a + b, e), sm::pow(a * c, e)).  4 (default): dense
-     * same-shape operands -- or one dense operand and a constant, for + - * -- run the pow kernel itself (float and
-     * double) with the operator applied to the loaded operands (bit-identical to the operator followed by sm::pow);
-     * everything else, and the values 0..3, use the general chain kernel --
-     * 0: one vector per thread, no prefetch (round 1); 1: one vector + register prefetch of the next tile's
-     * leaves; 2: two vectors; 3: two vectors + prefetch. */
-    SMB_OPT_CHAIN_POW_VARIANT = 11,
-    /* Device set: how an operand several devices read (or whose per-device ranges are below a page) reaches them.
-     * 0 (default): the operand is advised read-mostly and each device's range prefetched to it ONCE -- the driver keeps a
-     * read-only duplicate per device and invalidates them on any write (raw host writes included); 1: a private copy per
-     * call in pooled device scratch (subject to SMB_OPT_REPLICATE_MAX_BYTES). */
-    SMB_OPT_REPLICA_MODE = 12,
-    /* Device set, synchronous mode: 1 (default) every device of the set has a persistent launcher thread that prepares,
-     * launches and waits for its device's range, all devices at once; 0: the calling thread walks the devices. */
-    SMB_OPT_LAUNCHER_THREADS = 13
+    SMB_OPT_POOL_MAX_CACHED_BYTES = 9
+    /* 2, 3 and 10..13 are retired: setting one fails like any unknown option, and they are not reused. */
 };
 
 /* ---- the hot path ------------------------------------------------------- */
@@ -274,7 +250,7 @@ int smb_wait_pending(void);
  * operands and result are MANAGED blocks (the drop-in SMArray storage) and whose result is at least
  * SMB_OPT_SHARD_MIN_BYTES is spread over those devices from the calling thread: device g computes
  * flat range g of the result on its own stream, reading its ranges of the contiguous operands in
- * place (pages prefetched to it once, then remembered) and a private copy of shared operands.  The
+ * place (pages prefetched to it once, then remembered) and a read-mostly duplicate of shared operands.  The
  * caller still writes `a + b` and nothing else (reference include/SMArray.h:217-225).  count <= 1
  * restores single-device behaviour; a device listed k times owns k ranges.  The environment variable SMB_DEVICES ("all", "0-7", "0,2")
  * presets the set for unmodified programs.  Device blocks (SMB_MEM_DEVICE) are computed where they
@@ -311,7 +287,7 @@ int smb_plan_chain(const smb_chain_step *steps, int nsteps, const uint64_t *shap
 /* The multi-GPU planner alone (smb_set_devices acts on it): where the flat result range of an
  * smb_elementwise call is cut for `ndev` devices (out_bounds[ndev + 1]), which element range
  * [lo, hi) of each operand device g reads (out_range_x[2 g], [2 g + 1]) and how each operand reaches
- * the devices (out_modes: 0 in place -- the ranges are disjoint --, 1 replicated per device, 2 shared
+ * the devices (out_modes: 0 in place -- the ranges are disjoint --, 1 read-mostly duplicate per device, 2 shared
  * and larger than SMB_OPT_REPLICATE_MAX_BYTES).  Returns 1 when the call would be sharded, 0 when it
  * would run on one device, or a negative error. */
 int smb_plan_shards(const uint64_t *stride_a, const uint64_t *stride_b, const uint64_t *shape, int ndim,

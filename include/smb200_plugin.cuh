@@ -120,11 +120,11 @@ int launch_strided(const smb_launch_env *env, const void *a, const void *b, void
         const uint64_t nvec = t.count / (uint64_t)(vector_bytes / (int)sizeof(T));
         const unsigned grid = grid_for(nvec, (uint64_t)kBlock * UNROLL, env->sm_count, a_reused && b_reused ? 32 : 0);
         if (vector_bytes == 16) {
-            if (wide) k_row<T, Fn, 16, true, UNROLL, 0><<<grid, kBlock, 0, s>>>(pa, pb, po, t, a_reused, b_reused, 0u, fn);
-            else k_row<T, Fn, 16, false, UNROLL, 0><<<grid, kBlock, 0, s>>>(pa, pb, po, t, a_reused, b_reused, 0u, fn);
+            if (wide) k_row<T, Fn, 16, true, UNROLL><<<grid, kBlock, 0, s>>>(pa, pb, po, t, a_reused, b_reused, fn);
+            else k_row<T, Fn, 16, false, UNROLL><<<grid, kBlock, 0, s>>>(pa, pb, po, t, a_reused, b_reused, fn);
         } else {
-            if (wide) k_row<T, Fn, (int)sizeof(T), true, UNROLL, 0><<<grid, kBlock, 0, s>>>(pa, pb, po, t, a_reused, b_reused, 0u, fn);
-            else k_row<T, Fn, (int)sizeof(T), false, UNROLL, 0><<<grid, kBlock, 0, s>>>(pa, pb, po, t, a_reused, b_reused, 0u, fn);
+            if (wide) k_row<T, Fn, (int)sizeof(T), true, UNROLL><<<grid, kBlock, 0, s>>>(pa, pb, po, t, a_reused, b_reused, fn);
+            else k_row<T, Fn, (int)sizeof(T), false, UNROLL><<<grid, kBlock, 0, s>>>(pa, pb, po, t, a_reused, b_reused, fn);
         }
     }
     return (int)cudaGetLastError();

@@ -24,9 +24,15 @@ LIB_PATH = os.environ.get("SMB200_LIB") or os.path.join(HERE, "libsmb200.so")  #
 OP_ADD, OP_SUB, OP_MUL, OP_DIV, OP_POW = range(5)
 F32, F64, I32 = range(3)
 MEM_DEVICE, MEM_MANAGED, MEM_PINNED = range(3)
-(OPT_POW_SPECIALISE, OPT_STAGE_CHUNK_BYTES, OPT_CONTIG_VARIANT, OPT_BCAST_VARIANT, OPT_FORCE_WIDE_INDEX, OPT_ASYNC, OPT_PDL,
- OPT_SHARD_MIN_BYTES, OPT_REPLICATE_MAX_BYTES, OPT_POOL_MAX_CACHED_BYTES, OPT_POW_TAIL_CTAS, OPT_CHAIN_POW_VARIANT,
- OPT_REPLICA_MODE, OPT_LAUNCHER_THREADS) = range(14)
+# smb_set_option keys (include/smb200.h); 2, 3 and 10..13 are retired and not reused
+OPT_POW_SPECIALISE = 0
+OPT_STAGE_CHUNK_BYTES = 1
+OPT_FORCE_WIDE_INDEX = 4
+OPT_ASYNC = 5
+OPT_PDL = 6
+OPT_SHARD_MIN_BYTES = 7
+OPT_REPLICATE_MAX_BYTES = 8
+OPT_POOL_MAX_CACHED_BYTES = 9
 PLAN_CONTIGUOUS, PLAN_ROW, PLAN_GENERIC = range(3)
 MAX_NDIM = 6
 CHAIN_MAX = 8

@@ -103,13 +103,12 @@ static int chain_launch(DeviceCtx &c, const ChainPlan &p, const smb_chain_step *
             powfast = true;
         }
     }
-    const int powvar = (int)g_opt_chain_pow_variant.load();
-    // sm::pow(a (op) b, y) on dense same-shape arrays -- THE fused pow (SMB_OPT_CHAIN_POW_VARIANT = 4, the default): the
-    // pow kernel itself with the operator applied to the two loaded operands (k_stream<PowF32FnPre>), bit-identical to
-    // the operator followed by the pow kernel and at that kernel's speed; the general chain kernel below was
-    // instruction-bound at 4.4-4.7 TB/s whatever its shape (profiles/r2_chain_pow_sweep.md).
+    // sm::pow(a (op) b, y) on dense same-shape arrays -- THE fused pow: the pow kernel itself with the operator applied
+    // to the two loaded operands (k_stream<PowF32FnPre>), bit-identical to the operator followed by the pow kernel and at
+    // that kernel's speed; the general chain kernel below was instruction-bound at 4.4-4.7 TB/s whatever its shape
+    // (profiles/r2_chain_pow_sweep.md).
     if constexpr (std::is_same<T, float>::value) {
-        if (powvar == 4 && p.nleaf == 3 && p.ndim == 1 && data[0] && data[1] && !data[2] && steps[2].op == SMB_OP_POW && chain_pow_special<T>(steps[2]) < 0 &&
+        if (p.nleaf == 3 && p.ndim == 1 && data[0] && data[1] && !data[2] && steps[2].op == SMB_OP_POW && chain_pow_special<T>(steps[2]) < 0 &&
             p.stride[0][0] == 1 && p.stride[1][0] == 1 && steps[1].op != SMB_OP_POW && pow_f32_fast_ok(classify_exp(steps[2].value.f32))) {
             // (any length and alignment: launch_stream peels heads and tails exactly as it does for sm::pow itself)
             const float y = steps[2].value.f32;
@@ -135,7 +134,7 @@ static int chain_launch(DeviceCtx &c, const ChainPlan &p, const smb_chain_step *
     }
     // sm::pow(a (op) constant, y), op in + - *, on a dense array: the pow kernel with a one-operand pre-operator (PowF32FnPre1).
     if constexpr (std::is_same<T, float>::value) {
-        if (powvar == 4 && p.nleaf == 3 && p.ndim == 1 && data[0] && !data[1] && !data[2] && steps[2].op == SMB_OP_POW && chain_pow_special<T>(steps[2]) < 0 &&
+        if (p.nleaf == 3 && p.ndim == 1 && data[0] && !data[1] && !data[2] && steps[2].op == SMB_OP_POW && chain_pow_special<T>(steps[2]) < 0 &&
             p.stride[0][0] == 1 && steps[1].op != SMB_OP_POW && steps[1].op != SMB_OP_DIV && pow_f32_fast_ok(classify_exp(steps[2].value.f32))) {
             const float y = steps[2].value.f32, cst = steps[1].value.f32;
             const PowExpF32 pe = classify_exp(y);
@@ -158,7 +157,7 @@ static int chain_launch(DeviceCtx &c, const ChainPlan &p, const smb_chain_step *
     }
     // the same two shapes for double (PowF64FnPre / PowF64FnPre1)
     if constexpr (std::is_same<T, double>::value) {
-        const bool shape_ok = powvar == 4 && p.nleaf == 3 && p.ndim == 1 && data[0] && !data[2] && steps[2].op == SMB_OP_POW &&
+        const bool shape_ok = p.nleaf == 3 && p.ndim == 1 && data[0] && !data[2] && steps[2].op == SMB_OP_POW &&
                               chain_pow_special<T>(steps[2]) < 0 && p.stride[0][0] == 1 && steps[1].op != SMB_OP_POW;
         const bool two = shape_ok && data[1] && p.stride[1][0] == 1, one = shape_ok && !data[1] && steps[1].op != SMB_OP_DIV;
         if (two || one) {
@@ -185,24 +184,14 @@ static int chain_launch(DeviceCtx &c, const ChainPlan &p, const smb_chain_step *
             return rc;
         }
     }
-    t.tiles_per_cta = powfast ? (powvar == 2 || powvar == 3 ? 16 : 32) : 1; // amortise the 24 KB table copy, stay many waves deep
+    t.tiles_per_cta = powfast ? 32 : 1; // amortise the 24 KB table copy, stay many waves deep
     // compiled-in chain capacity / vectors per thread: short chains keep more loads in flight
 #define SMB_CHAIN_LAUNCH(E, W, NS, U, PF, ND)                                                                     \
     k_chain<T, E, W, NS, U, PF, ND><<<grid_for(items, (uint64_t)kThreads * U * t.tiles_per_cta, c.sm_count, 0), kThreads, 0, s>>>(out, t)
-#define SMB_CHAIN_LAUNCH_PF(E, W, U, ND, PRE)                                                                     \
-    k_chain<T, E, W, 3, U, true, ND, PRE><<<grid_for(items, (uint64_t)kThreads * U * t.tiles_per_cta, c.sm_count, 0), kThreads, 0, s>>>(out, t)
 #define SMB_CHAIN_BY_LEN(E, W, PF, ND)                                                            \
     do {                                                                                          \
-        if (p.nleaf <= 3 && PF) { /* sm::pow(a (op) b, e): vectors per thread x register prefetch, SMB_OPT_CHAIN_POW_VARIANT */ \
-            if constexpr (PF) {                                                                   \
-                switch (powvar) {                                                                 \
-                    case 0: SMB_CHAIN_LAUNCH_PF(E, W, 1, ND, false); break;                       \
-                    case 2: SMB_CHAIN_LAUNCH_PF(E, W, 2, ND, false); break;                       \
-                    case 3: SMB_CHAIN_LAUNCH_PF(E, W, 2, ND, true); break;                        \
-                    case 1: SMB_CHAIN_LAUNCH_PF(E, W, 1, ND, true); break;                        \
-                    default: SMB_CHAIN_LAUNCH_PF(E, W, 1, ND, false); break; /* what does not fit the fused pow kernel */ \
-                }                                                                                 \
-            }                                                                                     \
+        if (p.nleaf <= 3 && PF) { /* sm::pow(a (op) b, e) the fused pow kernel does not take: one vector per thread */ \
+            if constexpr (PF) SMB_CHAIN_LAUNCH(E, W, 3, 1, true, ND);                             \
         }                                                                                         \
         else if (p.nleaf <= 3) SMB_CHAIN_LAUNCH(E, W, 3, 4, PF, ND);                              \
         else if (p.nleaf <= 5) SMB_CHAIN_LAUNCH(E, W, 5, 2, PF, ND);                              \
@@ -230,7 +219,6 @@ static int chain_launch(DeviceCtx &c, const ChainPlan &p, const smb_chain_step *
     }
 #undef SMB_CHAIN_BY_RANK
 #undef SMB_CHAIN_BY_LEN
-#undef SMB_CHAIN_LAUNCH_PF
 #undef SMB_CHAIN_LAUNCH
     ++g_launches;
     note_other_op(); // a plain launch: the next stream kernel after it is launched plainly too
@@ -638,8 +626,6 @@ int smb_set_option(int key, int64_t value) {
     switch (key) {
         case SMB_OPT_POW_SPECIALISE: g_opt_pow_specialise = value ? 1 : 0; return SMB_OK;
         case SMB_OPT_STAGE_CHUNK_BYTES: g_opt_chunk_bytes = value; return SMB_OK;
-        case SMB_OPT_CONTIG_VARIANT: g_opt_contig_variant = value; return SMB_OK;
-        case SMB_OPT_BCAST_VARIANT: g_opt_bcast_variant = value; return SMB_OK;
         case SMB_OPT_FORCE_WIDE_INDEX: g_opt_force_wide = value ? 1 : 0; return SMB_OK;
         case SMB_OPT_ASYNC:
             if (!value && g_opt_async.load()) { g_opt_async = 0; return sync_all(); } // leaving async mode: everything lands
@@ -649,10 +635,6 @@ int smb_set_option(int key, int64_t value) {
         case SMB_OPT_SHARD_MIN_BYTES: g_opt_shard_min_bytes = value; return SMB_OK;
         case SMB_OPT_REPLICATE_MAX_BYTES: g_opt_replicate_max_bytes = value; return SMB_OK;
         case SMB_OPT_POOL_MAX_CACHED_BYTES: g_opt_pool_max_cached = value; return SMB_OK;
-        case SMB_OPT_POW_TAIL_CTAS: g_opt_pow_tail = value; return SMB_OK;
-        case SMB_OPT_CHAIN_POW_VARIANT: g_opt_chain_pow_variant = value; return SMB_OK;
-        case SMB_OPT_REPLICA_MODE: g_opt_replica_mode = value; return SMB_OK;
-        case SMB_OPT_LAUNCHER_THREADS: g_opt_launcher_threads = value ? 1 : 0; return SMB_OK;
     }
     return fail(SMB_ERR_INVALID, "unknown option %d", key);
 }
@@ -660,18 +642,12 @@ int64_t smb_get_option(int key) {
     switch (key) {
         case SMB_OPT_POW_SPECIALISE: return g_opt_pow_specialise;
         case SMB_OPT_STAGE_CHUNK_BYTES: return g_opt_chunk_bytes;
-        case SMB_OPT_CONTIG_VARIANT: return g_opt_contig_variant;
-        case SMB_OPT_BCAST_VARIANT: return g_opt_bcast_variant;
         case SMB_OPT_FORCE_WIDE_INDEX: return g_opt_force_wide;
         case SMB_OPT_ASYNC: return g_opt_async;
         case SMB_OPT_PDL: return g_opt_pdl;
         case SMB_OPT_SHARD_MIN_BYTES: return g_opt_shard_min_bytes;
         case SMB_OPT_REPLICATE_MAX_BYTES: return g_opt_replicate_max_bytes;
         case SMB_OPT_POOL_MAX_CACHED_BYTES: return g_opt_pool_max_cached;
-        case SMB_OPT_POW_TAIL_CTAS: return g_opt_pow_tail;
-        case SMB_OPT_CHAIN_POW_VARIANT: return g_opt_chain_pow_variant;
-        case SMB_OPT_REPLICA_MODE: return g_opt_replica_mode;
-        case SMB_OPT_LAUNCHER_THREADS: return g_opt_launcher_threads;
     }
     return -1;
 }

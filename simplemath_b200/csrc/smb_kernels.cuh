@@ -26,12 +26,6 @@ constexpr int kBlock = 256; // threads per CTA of every kernel in this file
 #ifndef SMB_STREAM_STORE_HINT
 #define SMB_STREAM_STORE_HINT true
 #endif
-#ifndef SMB_POW_BLOCKED
-#define SMB_POW_BLOCKED 1 // pow loop: consecutive tiles per CTA on a many-wave grid (0: resident grid, grid-stride)
-#endif
-#ifndef SMB_POW_PINGPONG
-#define SMB_POW_PINGPONG 1 // f32/f64 pow loop: swap the two tile buffers (unroll by two) instead of copying
-#endif
 // The pow tile body is one long basic block; without a fence ptxas sinks the next tile's loads
 // to its end (no prefetch left) and holds every store until then.  A warp-level barrier is one
 // instruction it will not move memory operations across.
@@ -134,8 +128,8 @@ template<typename T, int BYTES> union Pack {
 };
 
 // ---------------------------------------------------------------------------
-// mbarrier + 1-D bulk copy (TMA engine, SASS UBLKCP): used to stage the pow lookup tables and a
-// reused broadcast operand in shared memory with one instruction instead of a load/store loop.
+// mbarrier + 1-D bulk copy (TMA engine, SASS UBLKCP): used to stage the pow lookup tables in shared
+// memory with one instruction instead of a load/store loop.
 __device__ __forceinline__ uint32_t smem_addr(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_addr(bar)), "r"(count));
@@ -165,7 +159,6 @@ __device__ __forceinline__ void bulk_g2s(void *smem, const void *gmem, uint32_t 
 // completion still implies the previous one's).  Both instructions are no-ops in a launch without
 // the programmatic-stream-serialisation attribute.  The host side is in smb_runtime.inl (pdl_decide).
 constexpr uint32_t kPdlWaitFirst = 1u;
-constexpr int kPdlFlagBits = 8; // the launch word's upper 24 bits carry a kernel-specific count (k_stream: single-tile CTAs)
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 // A launch that must wait for its predecessors lets ITS dependents in only after the wait has returned: the host drops its
@@ -628,60 +621,29 @@ __global__ void __launch_bounds__(256, fn_pow_tables<Fn>::value ? (sizeof(T) == 
             if constexpr (PRE) pow_tile<T, Fn, VB, UNROLL, true>(BA, BB, a, b, out, (TILE) * tile_vecs + threadIdx.x, fn); \
             else pow_tile<T, Fn, VB, UNROLL, false>(BA, BA, a, a, out, (TILE) * tile_vecs + threadIdx.x, fn); \
         } while (0)
-#if SMB_POW_BLOCKED
         // CTA b owns `tpc` CONSECUTIVE tiles: the host sizes the grid so that tpc is a handful of tiles --
         // enough to amortise the table fill, few enough that the grid is many waves deep (a grid of
         // resident CTAs striding over everything measured 10-15 % slower on B200 for any 1-read-1-write
-        // stream: profiles/r1_sweep_summary.md).  The LAST `n_small` CTAs of the grid (the hardware hands
-        // CTAs out in index order, so they run last) own ONE tile each: multi-tile CTAs end raggedly, up
-        // to one CTA lifetime apart across the SMs, and single-tile CTAs fill those gaps -- what cost
-        // ~14 us per launch at the 8-GPU shard size (2^27 elements, a 170 us kernel).
-        const uint64_t n_small = pdl >> kPdlFlagBits;
-        const uint64_t n_big = gridDim.x - n_small, tiles_big = full_tiles - n_small; // host: n_small <= gridDim.x, full_tiles
-        const uint64_t tpc = n_big ? (tiles_big + n_big - 1) / n_big : 0, tstep = 1;
-        uint64_t tile, tiles_end;
-        if (blockIdx.x < n_big) {
-            tile = blockIdx.x * tpc;
-            tiles_end = tile + tpc < tiles_big ? tile + tpc : tiles_big;
-        } else {
-            tile = tiles_big + (blockIdx.x - n_big);
-            tiles_end = tile + 1;
-        }
-#else
-        const uint64_t tstep = gridDim.x, tiles_end = full_tiles;
-        uint64_t tile = blockIdx.x;
-#endif
+        // stream: profiles/r1_sweep_summary.md).
+        const uint64_t tpc = (full_tiles + gridDim.x - 1) / gridDim.x;
+        uint64_t tile = blockIdx.x * tpc;
+        const uint64_t tiles_end = tile + tpc < full_tiles ? tile + tpc : full_tiles;
         if (tile < tiles_end) { SMB_POW_LOAD_TILE(buf0, bb0, tile) }
         fn.block_wait(); // the tables have landed (the copy overlapped the loads above)
-#if SMB_POW_PINGPONG
 #pragma unroll 1
         while (tile < tiles_end) {
-            uint64_t next = tile + tstep;
+            uint64_t next = tile + 1;
             if (next < tiles_end) { SMB_POW_LOAD_TILE(buf1, bb1, next) }
             SMB_POW_SCHED_FENCE();
             SMB_POW_RUN_TILE(buf0, bb0, tile);
             tile = next;
             if (tile >= tiles_end) break;
-            next = tile + tstep;
+            next = tile + 1;
             if (next < tiles_end) { SMB_POW_LOAD_TILE(buf0, bb0, next) }
             SMB_POW_SCHED_FENCE();
             SMB_POW_RUN_TILE(buf1, bb1, tile);
             tile = next;
         }
-#else
-#pragma unroll 1
-        for (; tile < tiles_end; tile += tstep) {
-            const uint64_t next = tile + tstep;
-            if (next < tiles_end) { SMB_POW_LOAD_TILE(buf1, bb1, next) }
-            SMB_POW_SCHED_FENCE();
-            SMB_POW_RUN_TILE(buf0, bb0, tile);
-#pragma unroll
-            for (int u = 0; u < UNROLL; ++u) {
-                buf0[u].raw = buf1[u].raw;
-                if constexpr (PRE) bb0[u].raw = bb1[u].raw;
-            }
-        }
-#endif
 #undef SMB_POW_LOAD_TILE
 #undef SMB_POW_RUN_TILE
     } else {
@@ -776,37 +738,12 @@ __device__ __forceinline__ void offsets_of(const BcastTable &t, uint64_t lin, ui
 // issued before the first use.  An operand with inner stride 1 is read with one vector
 // load; with inner stride 0 with one scalar load that is splat.  Operands with any zero
 // stride are re-read by other threads, so they use the default (caching) load path; pure
-// streams use the streaming hints.
-//
-// STAGE = 1 / 2: operand a / b is small (its whole extent fits the shared-memory budget)
-// and reused -- it is staged in shared memory once per CTA (one cp.async.bulk when
-// 16-byte aligned, else a copy loop) and every later read of it is an LDS.  The grid is
-// persistent in that case so the staging is amortised.
-template<typename T, typename Fn, int VB, bool WIDE, int UNROLL, int STAGE>
+// streams use the streaming hints.  (Staging the reused operand in shared memory measured
+// slower on B200: DESIGN.md §4.2.)
+template<typename T, typename Fn, int VB, bool WIDE, int UNROLL>
 __global__ void __launch_bounds__(256) k_row(const T *__restrict__ a, const T *__restrict__ b, T *__restrict__ out,
-                                            const __grid_constant__ BcastTable t, int a_reused, int b_reused,
-                                            uint32_t stage_elems, Fn fn) {
+                                            const __grid_constant__ BcastTable t, int a_reused, int b_reused, Fn fn) {
     constexpr int EPV = VB / (int)sizeof(T);
-    extern __shared__ __align__(16) unsigned char k_row_smem[];
-    if constexpr (STAGE != 0) {
-        T *s_op = reinterpret_cast<T *>(k_row_smem + 16);
-        uint64_t *bar = reinterpret_cast<uint64_t *>(k_row_smem);
-        const T *src = STAGE == 1 ? a : b;
-        const uint32_t bytes = stage_elems * (uint32_t)sizeof(T);
-        if ((reinterpret_cast<uintptr_t>(src) & 15) == 0 && (bytes & 15) == 0) {
-            if (threadIdx.x == 0) {
-                mbar_init(bar, 1);
-                mbar_expect_tx(bar, bytes);
-                bulk_g2s(s_op, src, bytes, bar);
-            }
-            __syncthreads();
-            mbar_wait(bar, 0);
-        } else {
-            for (uint32_t i = threadIdx.x; i < stage_elems; i += kBlock) s_op[i] = src[i];
-            __syncthreads();
-        }
-        if (STAGE == 1) a = s_op; else b = s_op;
-    }
     const uint64_t nvec = t.count / EPV; // host guarantees count % EPV == 0 when EPV > 1
     const int m = t.ndim;
     const bool ia = t.sa[m - 1] != 0, ib = t.sb[m - 1] != 0;
@@ -824,16 +761,14 @@ __global__ void __launch_bounds__(256) k_row(const T *__restrict__ a, const T *_
                     pb[u].e[0] = b[ob];
                 } else {
                     if (ia) {
-                        if (STAGE == 1) pa[u].raw = *reinterpret_cast<const RawVec<VB> *>(a + oa);
-                        else pa[u].raw = a_reused ? VecIO<VB, false>::load(a + oa) : VecIO<VB, true>::load(a + oa);
+                        pa[u].raw = a_reused ? VecIO<VB, false>::load(a + oa) : VecIO<VB, true>::load(a + oa);
                     } else {
                         const T s = a[oa];
 #pragma unroll
                         for (int k = 0; k < EPV; ++k) pa[u].e[k] = s;
                     }
                     if (ib) {
-                        if (STAGE == 2) pb[u].raw = *reinterpret_cast<const RawVec<VB> *>(b + ob);
-                        else pb[u].raw = b_reused ? VecIO<VB, false>::load(b + ob) : VecIO<VB, true>::load(b + ob);
+                        pb[u].raw = b_reused ? VecIO<VB, false>::load(b + ob) : VecIO<VB, true>::load(b + ob);
                     } else {
                         const T s = b[ob];
 #pragma unroll
@@ -1121,9 +1056,7 @@ template<typename T> __device__ __noinline__ T chain_sqrt(T a) {
 // index and offset loops are then straight-line code on constant-bank operands -- with the rank a
 // run-time value the guarded 6-dim loops were 58 instructions per element, most of them IMAD / MOV /
 // ISETP / BRA), 0: any rank, guarded loops.
-// PIN: the vector loads are ordinary coherent loads with a memory clobber, which ptxas keeps where they are
-// written (a prefetch issued a whole tile ahead is otherwise sunk down to its first use, see pow_tile).
-template<typename T, int EPV, bool WIDE, int NS, int UNROLL, int NDIM, bool PIN = false>
+template<typename T, int EPV, bool WIDE, int NS, int UNROLL, int NDIM>
 __device__ __forceinline__ void chain_load(const ChainTable &t, uint64_t tile, uint64_t nvec, T (&leaf)[UNROLL][NS][EPV]) {
     using Idx = typename std::conditional<WIDE, uint64_t, uint32_t>::type;
     constexpr int KMAX = NDIM ? NDIM : SMB_MAX_NDIM;
@@ -1159,8 +1092,7 @@ __device__ __forceinline__ void chain_load(const ChainTable &t, uint64_t tile, u
                         if (k < ndim) off += (uint64_t)idx[k] * t.stride[s][k];
                     if (EPV > 1 && t.stride[s][ndim - 1] == 1) {
                         Pack<T, 16> pk; // EPV * sizeof(T) == 16
-                        if constexpr (PIN) pk.raw = load_stream_pinned(reinterpret_cast<const RawVec<16> *>(base + off));
-                        else pk.raw = VecIO<16, false>::load(base + off);
+                        pk.raw = VecIO<16, false>::load(base + off);
 #pragma unroll
                         for (int e = 0; e < EPV; ++e) leaf[u][s][e] = pk.e[e];
                     } else {
@@ -1271,7 +1203,7 @@ __device__ __forceinline__ void chain_compute(const ChainTable &t, uint64_t tile
 // first tile's loads) and a pow step goes through the FFMA2 core, two elements per call, the
 // reference-accuracy path only for the vectors it declines -- sm::pow(a + b, e) in one pass.  Such a
 // CTA runs several consecutive tiles to amortise the copy; plain chains run one tile per CTA.
-template<typename T, int EPV, bool WIDE, int NS, int UNROLL, bool POWFAST, int NDIM, bool PREFETCH = false>
+template<typename T, int EPV, bool WIDE, int NS, int UNROLL, bool POWFAST, int NDIM>
 __global__ void __launch_bounds__(256) k_chain(T *__restrict__ out, const __grid_constant__ ChainTable t) {
     const uint64_t nvec = t.count / EPV; // host guarantees count % EPV == 0
     const uint64_t ntiles = (nvec + kBlock * UNROLL - 1) / (kBlock * UNROLL);
@@ -1296,39 +1228,19 @@ __global__ void __launch_bounds__(256) k_chain(T *__restrict__ out, const __grid
             mbar_wait(&tab_bar, 0);
             return;
         }
-        if constexpr (PREFETCH) {
-            // The pow step is ~120 issue slots per vector: with the NEXT tile's leaf loads issued before this
-            // tile's arithmetic (two leaf buffers swapping roles) HBM latency hides under the warp's own
-            // math instead of relying on the other resident warps (sm::pow(a + b, e): 4.4 -> see profiles/).
-            T leaf0[UNROLL][NS][EPV], leaf1[UNROLL][NS][EPV];
-            chain_load<T, EPV, WIDE, NS, UNROLL, NDIM, true>(t, tile, nvec, leaf0);
-            mbar_wait(&tab_bar, 0); // the tables have landed (the copy overlapped the loads above)
-            asm volatile("" : "+r"(lane.log_off), "+r"(lane.exp_off) :: "memory"); // ties the lookups to the wait
+        // Occupancy (one vector per thread, four CTAs) hides the leaf loads; a register prefetch of the next tile
+        // measured slower (profiles/r2_chain_pow_sweep.jsonl).
+        bool first = true;
 #pragma unroll 1
-            while (tile < tile_end) {
-                if (tile + 1 < tile_end) chain_load<T, EPV, WIDE, NS, UNROLL, NDIM, true>(t, tile + 1, nvec, leaf1);
-                SMB_POW_SCHED_FENCE();
-                chain_compute<T, EPV, NS, UNROLL, true>(t, tile, nvec, leaf0, out, lane);
-                if (++tile >= tile_end) break;
-                if (tile + 1 < tile_end) chain_load<T, EPV, WIDE, NS, UNROLL, NDIM, true>(t, tile + 1, nvec, leaf0);
-                SMB_POW_SCHED_FENCE();
-                chain_compute<T, EPV, NS, UNROLL, true>(t, tile, nvec, leaf1, out, lane);
-                ++tile;
+        for (; tile < tile_end; ++tile) {
+            T leaf[UNROLL][NS][EPV];
+            chain_load<T, EPV, WIDE, NS, UNROLL, NDIM>(t, tile, nvec, leaf);
+            if (first) {
+                mbar_wait(&tab_bar, 0); // the tables have landed (the copy overlapped the loads above)
+                asm volatile("" : "+r"(lane.log_off), "+r"(lane.exp_off) :: "memory"); // ties the lookups to the wait
+                first = false;
             }
-        } else {
-            // No register prefetch: occupancy (one vector per thread, four CTAs) hides the loads instead.
-            bool first = true;
-#pragma unroll 1
-            for (; tile < tile_end; ++tile) {
-                T leaf[UNROLL][NS][EPV];
-                chain_load<T, EPV, WIDE, NS, UNROLL, NDIM>(t, tile, nvec, leaf);
-                if (first) {
-                    mbar_wait(&tab_bar, 0); // the tables have landed (the copy overlapped the loads above)
-                    asm volatile("" : "+r"(lane.log_off), "+r"(lane.exp_off) :: "memory"); // ties the lookups to the wait
-                    first = false;
-                }
-                chain_compute<T, EPV, NS, UNROLL, true>(t, tile, nvec, leaf, out, lane);
-            }
+            chain_compute<T, EPV, NS, UNROLL, true>(t, tile, nvec, leaf, out, lane);
         }
     }
 }

@@ -262,30 +262,27 @@ def test_staging_pipeline_many_chunks(orc):
         smb.set_option(smb.OPT_STAGE_CHUNK_BYTES, 64 << 20)
 
 
-def test_shared_memory_staged_broadcast_variant(orc):
-    """SMB_OPT_BCAST_VARIANT=1: the small reused operand is staged in shared memory
-    (cp.async.bulk when aligned, copy loop otherwise); same bits as the default path."""
+def test_reused_broadcast_operand_vector_row_kernel(orc):
+    """A small reused operand (a row, a column, a 4-D view's small factor) is read through L1/L2 by
+    the row kernel (k_row<vec16> for the aligned rows); same bits as the oracle."""
     rng = np.random.default_rng(21)
-    smb.set_option(smb.OPT_BCAST_VARIANT, 1)
-    try:
-        a = rng.standard_normal((300, 1024)).astype(np.float32)
-        row = rng.standard_normal((1, 1024)).astype(np.float32)
-        assert_same_bits(smb.binary("add", a, row), orc.binary("add", a, row), "stage b (bulk copy)")
-        assert smb.last_kernel() == "k_row<vec16,stage_b>"
-        assert_same_bits(smb.binary("sub", row, a), orc.binary("sub", row, a), "stage a")
-        assert smb.last_kernel() == "k_row<vec16,stage_a>"
-        big = rng.integers(-99, 99, size=(4, 64, 20, 4)).astype(np.int32)
-        small = rng.integers(1, 9, size=(1, 64, 1, 4)).astype(np.int32)
-        assert_same_bits(smb.binary("mul", big[2], small), orc.binary("mul", big[2], small), "4-D view, staged small operand")
-        col = rng.standard_normal((300, 1)).astype(np.float32)
-        assert_same_bits(smb.binary("mul", a, col), orc.binary("mul", a, col), "inner-broadcast operand staged")
-    finally:
-        smb.set_option(smb.OPT_BCAST_VARIANT, 0)
+    a = rng.standard_normal((300, 1024)).astype(np.float32)
+    row = rng.standard_normal((1, 1024)).astype(np.float32)
+    assert_same_bits(smb.binary("add", a, row), orc.binary("add", a, row), "reused b")
+    assert smb.last_kernel() == "k_row<vec16>"
+    assert_same_bits(smb.binary("sub", row, a), orc.binary("sub", row, a), "reused a")
+    assert smb.last_kernel() == "k_row<vec16>"
+    big = rng.integers(-99, 99, size=(4, 64, 20, 4)).astype(np.int32)
+    small = rng.integers(1, 9, size=(1, 64, 1, 4)).astype(np.int32)
+    assert_same_bits(smb.binary("mul", big[2], small), orc.binary("mul", big[2], small), "4-D view, small reused operand")
+    col = rng.standard_normal((300, 1)).astype(np.float32)
+    assert_same_bits(smb.binary("mul", a, col), orc.binary("mul", a, col), "inner-broadcast reused operand")
 
 
-def test_outer_broadcast_kernel(orc):
+def test_outer_broadcast_kernel_and_row_fallback(orc):
     """{D0,1,L} (op) {1,D1,L} (config C4's pattern) takes the register-tiled k_outer kernel:
-    both operand orders, non-commutative ops, ragged tile edges, slab-aligned shards."""
+    both operand orders, non-commutative ops, ragged tile edges, slab-aligned shards; rows that
+    are not vector-aligned and ranges that are not whole slabs fall back to k_row, same bits."""
     torch = _torch()
     rng = np.random.default_rng(41)
     for d0, d1, L in ((5, 7, 40), (16, 16, 1024), (3, 130, 12), (33, 2, 2052)):
@@ -298,7 +295,7 @@ def test_outer_broadcast_kernel(orc):
             assert smb.last_kernel() == "k_outer<4x4>"
         xf, yf = x.astype(np.float64), y.astype(np.float64)
         assert_same_bits(smb.binary("div", xf, yf), orc.binary("div", xf, yf), "outer f64")
-    # not vector-aligned rows -> k_row; disabled by option -> k_row; results identical
+    # not vector-aligned rows -> k_row; results identical
     x = rng.integers(-9, 9, size=(6, 1, 37)).astype(np.int32)
     y = rng.integers(1, 9, size=(1, 5, 37)).astype(np.int32)
     assert_same_bits(smb.binary("mul", x, y), orc.binary("mul", x, y), "odd row length")
@@ -314,12 +311,6 @@ def test_outer_broadcast_kernel(orc):
         smb.elementwise_range_ptr(smb.OP_SUB, smb.F32, dx.data_ptr(), sa, dy.data_ptr(), sb, shape, lo, cnt, part.data_ptr())
         assert smb.last_kernel().startswith(kern), (lo, cnt, smb.last_kernel())
         assert_same_bits(part.cpu().numpy(), want[lo:lo + cnt], f"range {lo}+{cnt}")
-    smb.set_option(smb.OPT_BCAST_VARIANT, 2)
-    try:
-        assert_same_bits(smb.binary("sub", x, y), orc.binary("sub", x, y), "outer kernel disabled")
-        assert smb.last_kernel().startswith("k_row")
-    finally:
-        smb.set_option(smb.OPT_BCAST_VARIANT, 0)
 
 
 def test_outer_int_division_by_reciprocal_full_range(orc):

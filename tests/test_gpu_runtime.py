@@ -5,7 +5,7 @@
   * multi-GPU behind the operator API (smb_set_devices, SURVEY.md §8e): every operator spread over a
     device set, bit-identical to one device.  On a one-GPU box the set lists device 0 several times
     (each entry owns a flat range), which drives the whole sharded path -- range planning, placement
-    records, replicated operands, rebased pointers, per-range launches; with >= 2 GPUs the same tests
+    records, read-mostly duplicates of shared operands, per-range launches; with >= 2 GPUs the same tests
     also run on distinct devices;
   * asynchronous hand-off (SMB_OPT_ASYNC), programmatic dependent launch on / off;
   * the exhaustive device-side pow audit.
@@ -175,7 +175,7 @@ def test_sharded_elementwise_bit_identical(orc, sharded):
 
 
 def test_sharded_transposed_operand_falls_back_to_one_device(orc, sharded):
-    """An operand every device would need most of (a transpose) and that is too large to copy per call:
+    """An operand every device would need most of (a transpose) and that is too large to duplicate:
     the operator runs on one device -- same bits."""
     rng = np.random.default_rng(5)
     smb.set_devices([0, 0, 0, 0])
@@ -216,7 +216,7 @@ def test_sharded_scalar_pow_chain_fill_dot(orc, sharded):
         finally:
             smb.set_option(smb.OPT_POW_SPECIALISE, 1)
         assert oracle.ulp_error_f32(mo.np.copy(), orc.pow_ref_f32(x, 2.5)).max() <= 0.6
-        # fused chain with a broadcast row leaf (replicated) and a column leaf
+        # fused chain with a broadcast row leaf (shared: read-mostly duplicates) and a column leaf
         a = rng.standard_normal((300, 256)).astype(np.float32)
         row = rng.standard_normal((1, 256)).astype(np.float32)
         col = rng.standard_normal((300, 1)).astype(np.float32)
@@ -267,6 +267,28 @@ def test_sharded_reuses_placement_and_results_feed_the_next_operator(orc, sharde
     smb.lib().smb_host_written(ma.ptr)
     smb.elementwise_ptr(smb.OP_ADD, smb.F32, ma.ptr, full, mb.ptr, full, [R, C], mc.ptr)
     assert_same_bits(mc.np.copy(), orc.binary("add", b, b), "operand rewritten by the host between operators")
+
+
+def test_sharded_shared_operand_sees_raw_host_writes(orc, sharded):
+    """A shared operand (a broadcast row every device reads) is kept as read-mostly duplicates, which the driver
+    invalidates on any write: after the host rewrites the row through its pointer WITHOUT smb_host_written (as
+    SMArray::data allows), the next result sees the new values on every device."""
+    rng = np.random.default_rng(80)
+    R, C = 4096, 2048
+    a = rng.standard_normal((R, C)).astype(np.float32)
+    row = rng.standard_normal((1, C)).astype(np.float32)
+    ma, mr, mo = Managed(a), Managed(row), Managed(shape=a.shape, dtype=np.float32)
+    full, rowst = [C, 1], [0, 1]
+    for devs in _device_sets():
+        smb.set_devices(devs)
+        assert smb.plan_shards(full, rowst, [R, C], len(devs))[4][1] == 1  # the row: a read-mostly duplicate per device
+        for _ in range(2):  # the second call finds the partition and the duplicates in place
+            smb.elementwise_ptr(smb.OP_ADD, smb.F32, ma.ptr, full, mr.ptr, rowst, [R, C], mo.ptr)
+        assert_same_bits(mo.np.copy(), orc.binary("add", a, row), f"{len(devs)} ranges, row as first written")
+        row = rng.standard_normal((1, C)).astype(np.float32)
+        mr.np[...] = row
+        smb.elementwise_ptr(smb.OP_ADD, smb.F32, ma.ptr, full, mr.ptr, rowst, [R, C], mo.ptr)
+        assert_same_bits(mo.np.copy(), orc.binary("add", a, row), f"{len(devs)} ranges, row rewritten raw by the host")
 
 
 # ------------------------------------------------------------- async hand-off, PDL on / off ----

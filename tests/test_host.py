@@ -52,6 +52,21 @@ def test_product_never_imports_the_oracle():
             assert "liboracle" not in txt and "oracle/" not in txt.replace("oracle/oracle.c:orc_fill_uniform_f32", ""), f
 
 
+def test_retired_option_keys_are_rejected():
+    """Keys 2, 3 and 10..13 selected kernel variants and launch modes that measured slower and were removed:
+    setting one fails like any unknown key, reading one returns -1, and the keys that remain keep their numbers."""
+    lib = smb.lib()
+    for key in (2, 3, 10, 11, 12, 13):
+        assert lib.smb_set_option(key, 1) == 1  # SMB_ERR_INVALID
+        assert b"unknown option" in lib.smb_last_error()
+        with pytest.raises(smb.SmbError, match="unknown option"):
+            smb.set_option(key, 0)
+        assert lib.smb_get_option(key) == -1
+    assert (smb.OPT_POW_SPECIALISE, smb.OPT_STAGE_CHUNK_BYTES, smb.OPT_FORCE_WIDE_INDEX, smb.OPT_ASYNC, smb.OPT_PDL,
+            smb.OPT_SHARD_MIN_BYTES, smb.OPT_REPLICATE_MAX_BYTES, smb.OPT_POOL_MAX_CACHED_BYTES) == (0, 1, 4, 5, 6, 7, 8, 9)
+    assert lib.smb_get_option(smb.OPT_POW_SPECIALISE) == 1
+
+
 # ---- broadcast mirror ----------------------------------------------------------
 CASES = [((4096, 4096), (1, 4096)), ((512, 1, 1024), (1, 512, 1024)), ((224, 224, 3), (1, 224, 1, 3)),
          ((5,), (1,)), ((3, 1, 4, 1, 5), (2, 1, 6, 1)), ((1, 1), (1, 1)), ((7,), (3, 7)), ((2, 3, 4, 5, 6, 7), (7,))]

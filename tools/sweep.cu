@@ -167,7 +167,7 @@ struct PowLoopOnlyFn {
 template<int VB, int UNROLL>
 static void run_pow_loop_only(const float *a, float *out, uint64_t n) {
     const int caps[] = {1, 2, 4, 8, 16, 32, 64, 128};
-    for (int cap : caps) { // cap = tiles per CTA (SMB_POW_BLOCKED)
+    for (int cap : caps) { // cap = consecutive tiles per CTA, as the library's pow launch sizes them
         constexpr uint64_t per_block = 256ull * UNROLL * (VB / 4);
         uint64_t blocks = (n + per_block - 1) / per_block;
         blocks = (blocks + cap - 1) / cap;
@@ -181,7 +181,7 @@ static void run_pow_loop_only(const float *a, float *out, uint64_t n) {
 template<int VB, int UNROLL, bool SMALL>
 static void run_pow(const float *a, float *out, uint64_t n, float y) {
     const int caps[] = {1, 2, 4, 8, 16, 32, 64, 128};
-    for (int cap : caps) { // cap = tiles per CTA (SMB_POW_BLOCKED)
+    for (int cap : caps) { // cap = consecutive tiles per CTA, as the library's pow launch sizes them
         constexpr uint64_t per_block = 256ull * UNROLL * (VB / 4);
         uint64_t blocks = (n + per_block - 1) / per_block;
         blocks = (blocks + cap - 1) / cap;
@@ -224,32 +224,27 @@ static void run_tma(const float *a, const float *b, float *out, uint64_t n) {
     }
 }
 
-template<typename T, int OP, int UNROLL, int STAGE>
+template<typename T, int OP, int UNROLL>
 static void run_row_variant(const char *name, const T *a, const T *b, T *out, const ElementwisePlan &p, const BcastTable &t,
                             double bytes) {
     using Fn = BinaryFn<OP, T>;
     auto reused = [&](const uint64_t *s) { for (int k = 0; k < p.ndim; ++k) if (s[k] == 0 && p.shape[k] > 1) return 1; return 0; };
     const int ar = reused(p.sa), br = reused(p.sb);
-    const uint64_t ext = STAGE == 1 ? p.extent_a : p.extent_b;
-    const size_t smem = STAGE ? 16 + ext * sizeof(T) : 0;
-    if (smem > 200 * 1024) return;
-    if (STAGE) CK(cudaFuncSetAttribute(k_row<T, Fn, 16, false, UNROLL, STAGE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int caps[] = {0, 4, 8, 16, 32};
     for (int cap : caps) {
-        if (STAGE && cap == 0) continue;
         uint64_t nvec = p.n / (16 / sizeof(T));
         uint64_t blocks = (nvec + 256 * UNROLL - 1) / (256 * UNROLL);
         if (cap) blocks = std::min<uint64_t>(blocks, (uint64_t)g_sms * cap);
-        float ms = time_ms([&] { k_row<T, Fn, 16, false, UNROLL, STAGE><<<(unsigned)blocks, 256, smem>>>(a, b, out, t, ar, br, (uint32_t)ext, Fn{0}); });
+        float ms = time_ms([&] { k_row<T, Fn, 16, false, UNROLL><<<(unsigned)blocks, 256>>>(a, b, out, t, ar, br, Fn{0}); });
         char pr[128];
-        snprintf(pr, sizeof pr, "vec16 unroll=%d stage=%d ctas_per_sm=%d", UNROLL, STAGE, cap);
+        snprintf(pr, sizeof pr, "vec16 unroll=%d ctas_per_sm=%d", UNROLL, cap);
         report(name, pr, bytes, ms);
     }
 }
 
 template<typename T, int OP>
 static void run_row(const char *name, const T *a, const T *b, T *out, const uint64_t *shape, const uint64_t *sa, const uint64_t *sb,
-                    int ndim, double bytes, bool try_stage_b) {
+                    int ndim, double bytes) {
     ElementwisePlan p = make_plan(sa, sb, shape, ndim);
     BcastTable t;
     memset(&t, 0, sizeof t);
@@ -263,13 +258,9 @@ static void run_row(const char *name, const T *a, const T *b, T *out, const uint
         t.shape[k] = f.d; t.mul[k] = f.mul; t.shr[k] = f.shr;
     }
     t.lin_base = 0; t.count = p.n; t.lane_base = 0;
-    run_row_variant<T, OP, 1, 0>(name, a, b, out, p, t, bytes);
-    run_row_variant<T, OP, 2, 0>(name, a, b, out, p, t, bytes);
-    run_row_variant<T, OP, 4, 0>(name, a, b, out, p, t, bytes);
-    if (try_stage_b) {
-        run_row_variant<T, OP, 1, 2>(name, a, b, out, p, t, bytes);
-        run_row_variant<T, OP, 4, 2>(name, a, b, out, p, t, bytes);
-    }
+    run_row_variant<T, OP, 1>(name, a, b, out, p, t, bytes);
+    run_row_variant<T, OP, 2>(name, a, b, out, p, t, bytes);
+    run_row_variant<T, OP, 4>(name, a, b, out, p, t, bytes);
 }
 
 int main(int argc, char **argv) {
@@ -346,19 +337,19 @@ int main(int argc, char **argv) {
     if (want("row")) {
         { // C2: f32 {4096,4096} + {1,4096}
             const uint64_t shape[2] = {4096, 4096}, sa[2] = {4096, 1}, sb[2] = {0, 1};
-            run_row<float, OP_ADD>("c2_row_add_f32", a, b, out, shape, sa, sb, 2, 4.0 * (2 * 16777216.0 + 4096), true);
+            run_row<float, OP_ADD>("c2_row_add_f32", a, b, out, shape, sa, sb, 2, 4.0 * (2 * 16777216.0 + 4096));
         }
         { // C2 scaled up to 1 GiB so it is not L2-resident: {65536,4096} + {1,4096}
             const uint64_t shape[2] = {65536, 4096}, sa[2] = {4096, 1}, sb[2] = {0, 1};
-            if (n >= (1ull << 28)) run_row<float, OP_ADD>("c2x16_row_add_f32", a, b, out, shape, sa, sb, 2, 4.0 * (2 * 268435456.0 + 4096), true);
+            if (n >= (1ull << 28)) run_row<float, OP_ADD>("c2x16_row_add_f32", a, b, out, shape, sa, sb, 2, 4.0 * (2 * 268435456.0 + 4096));
         }
         { // C4: i32 {512,1,1024} * {1,512,1024}
             const uint64_t shape[3] = {512, 512, 1024}, sa[3] = {1024, 0, 1}, sb[3] = {0, 1024, 1};
             if (n >= (1ull << 28)) {
-                run_row<int32_t, OP_MUL>("c4_row_mul_i32", (const int32_t *)a, (const int32_t *)b, (int32_t *)out, shape, sa, sb, 3, 4.0 * (268435456.0 + 2 * 524288), false);
+                run_row<int32_t, OP_MUL>("c4_row_mul_i32", (const int32_t *)a, (const int32_t *)b, (int32_t *)out, shape, sa, sb, 3, 4.0 * (268435456.0 + 2 * 524288));
                 k_fill<uint32_t><<<g_sms * 8, 256>>>((uint32_t *)b, 524288, 7u);
                 CK(cudaDeviceSynchronize());
-                run_row<int32_t, OP_DIV>("c4_row_div_i32", (const int32_t *)a, (const int32_t *)b, (int32_t *)out, shape, sa, sb, 3, 4.0 * (268435456.0 + 2 * 524288), false);
+                run_row<int32_t, OP_DIV>("c4_row_div_i32", (const int32_t *)a, (const int32_t *)b, (int32_t *)out, shape, sa, sb, 3, 4.0 * (268435456.0 + 2 * 524288));
             }
         }
     }
